@@ -5,6 +5,7 @@
     python bench.py --impl reference --gpus 1 --steps 3 --warmup 1      # the CPU path (oracle port)
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
            --master-port P bench.py --gpus N --steps K --warmup W       # N independent streams, 1/GPU
+    python bench.py --steps 10 --warmup 3 --dump-outputs DIR            # + the last timed step's results as DIR/*.npy
 
 Metric (BASELINE.json): stream audio-seconds per second = chunks/s x 0.5 s, 5 s windows @ 16 kHz,
 0.5 s step, batch 256.  A step is one pass of the fused pipeline (segmentation -> OSP -> embedding ->
@@ -26,6 +27,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark runs from a tree it must leave as it found it (possibly read-only)
 
 CHUNK, STEP, SR = 80000, 8000, 16000
 STEP_SECONDS = STEP / SR
@@ -149,6 +151,33 @@ def make_stream_batches(rank: int, n_batches: int, batch: int) -> np.ndarray:
     return np.stack([synth.windows(stream, batch, first=j * batch) for j in range(n_batches)])
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(directory: str, arrays: dict):
+    """Writes what the timed path returned in its last step, {name: array with windows on axis 0}, as directory/<name>.npy in
+    float32 (float64 arrays stay float64).  When that exceeds DUMP_LIMIT_BYTES in all, every array keeps the same seeded sample
+    of windows, whose indices are written as window_index.npy."""
+    arrays = {k: np.asarray(v, dtype=np.float64 if np.asarray(v).dtype == np.float64 else np.float32) for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    per_window = sum(a.nbytes for a in arrays.values()) // n + 8
+    if n * per_window > DUMP_LIMIT_BYTES - 4096:          # (4096: room for the .npy headers)
+        keep = np.sort(np.random.default_rng(0).choice(n, (DUMP_LIMIT_BYTES - 4096) // per_window, replace=False))
+        arrays = {k: a[keep] for k, a in arrays.items()}
+        arrays["window_index"] = keep.astype(np.float64)
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, f"{name}.npy"), a)
+
+
+def device_view(address: int, shape, typestr: str, device: torch.device) -> torch.Tensor:
+    """a tensor over a device buffer the library owns (no copy; valid as long as the library keeps the buffer)"""
+    class View:
+        __cuda_array_interface__ = {"shape": tuple(shape), "typestr": typestr, "data": (address, False), "version": 2}
+
+    return torch.as_tensor(View(), device=device)
+
+
 # ------------------------------------------------------------------------------------ reference arm
 def run_reference(args):
     """The reference's CPU path (oracle port: reference diart block logic restated in oracle/, torch-CPU
@@ -169,8 +198,11 @@ def run_reference(args):
         pipe(data[(i % nb) * rb:(i % nb + 1) * rb])
     t0 = time.perf_counter()
     for i in range(args.steps):
-        pipe(data[(i % nb) * rb:(i % nb + 1) * rb])
+        out = pipe(data[(i % nb) * rb:(i % nb + 1) * rb])
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        seg, emb, maps, margins = out
+        dump_outputs(args.dump_outputs, {"segmentation": seg, "embeddings": emb, "speaker_map": maps, "margins": margins})
     value = args.steps * rb * STEP_SECONDS / dt
     sample = f"{args.steps} steps x {rb} consecutive windows (of the batch-256 workload), K-fold repeated trunk as the reference runs it"
     line = {
@@ -266,20 +298,25 @@ def run_ours(args):
     stream = _lib.stream_ptr(device)
 
     shared = None
+    seg_p, emb_p, map_p = C.c_void_p(), C.c_void_p(), C.c_void_p()
 
     def run_steps(n):
         """n pipeline steps through dg_pipeline_submit / collect: the clustering of step i overlaps the networks of steps
-        i+1, i+2; every step's results are complete when the last collect is reached on the stream"""
+        i+1, i+2; every step's results are complete when the last collect is reached on the stream.  The last step's results:
+        serial, the returned (segmentation, embeddings, speaker map) device tensors; pipelined, the device pointers left in
+        seg_p / emb_p / map_p (the handle's slot buffers, valid until the third next submit)"""
         if args.serial:
+            out = None
             for i in range(n):
-                pipe.device_step(dev[i % NB])
-            return
+                out = pipe.device_step(dev[i % NB])
+            return out
+        collect = lambda: _lib.check(lib.dg_pipeline_collect(fused, C.byref(seg_p), C.byref(emb_p), C.byref(map_p), stream))
         for i in range(n):           # three steps outstanding, like the host-buffer leg
             _lib.check(lib.dg_pipeline_submit(fused, dev[i % NB].data_ptr(), B, CHUNK, stream))
             if i > 1:
-                _lib.check(lib.dg_pipeline_collect(fused, None, None, None, stream))
+                collect()
         for _ in range(min(n, 2)):
-            _lib.check(lib.dg_pipeline_collect(fused, None, None, None, stream))
+            collect()
 
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     with ClockSampler(local) as clocks:
@@ -289,11 +326,16 @@ def run_ours(args):
         launches0 = lib.dg_launch_count()
         clocks.mark()
         ev0.record()
-        run_steps(args.steps)
+        last = run_steps(args.steps)
         ev1.record()
         torch.cuda.synchronize(device)
         lib.dg_profile_enable(0)
         launches = lib.dg_launch_count() - launches0
+        if args.dump_outputs and rank == 0:      # copied before any further step reuses the slot buffers
+            if last is None:
+                last = (device_view(seg_p.value, (B, F, K), "<f4", device), device_view(emb_p.value, (B, K, D), "<f4", device),
+                        device_view(map_p.value, (B, K), "<i4", device))
+            dump_outputs(args.dump_outputs, dict(zip(("segmentation", "embeddings", "speaker_map"), (t.cpu().numpy() for t in last))))
         t_wait = time.monotonic()
         while not clocks.rows and clocks.proc is not None and time.monotonic() - t_wait < 3.0:
             run_steps(args.steps)            # nvidia-smi has not delivered a line yet: keep the same load until it does (untimed)
@@ -452,7 +494,7 @@ def run_ours(args):
         pipe.reset()
         sw_of = lambda n: SlidingWindow(start=STEP_SECONDS * n, duration=1 / SR, step=1 / SR)
         rows = [[np.ascontiguousarray(host[j][b][:, None]) for b in range(B)] for j in range(NB)]
-        n_calls = max(3, min(args.steps, 10))
+        n_calls = args.steps
 
         def call_steps(n, first):
             """the timed bracket is the reference's: `pipeline(batch)` only (inference.py:130-137); the batch objects exist before"""
@@ -709,7 +751,12 @@ def _main():
     ap.add_argument("--shared-identity", action="store_true",
                     help="BASELINE config 5: share the global speaker table across ranks (one all-gather per step)")
     ap.add_argument("--serial", action="store_true", help="one step at a time (dg_pipeline_step) instead of depth-2 pipelining")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step (segmentation, embeddings, speaker map) as DIR/<name>.npy; "
+                         "the inputs are seeded, so runs with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if args.impl == "reference":
         run_reference(args)
     else:
